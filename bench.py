@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- update-iteration throughput of the DPVO hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config default|fast]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config default|fast] [--dump-outputs DIR]
 
 One "step" = one DPVO.update() (dpvo/dpvo.py:328-360): reprojection, 2-level patch correlation,
 update operator, 2 Gauss-Newton BA iterations, on the steady-state synthetic patch graph of
@@ -19,6 +19,8 @@ HBM fraction) next to the DRAM and L2 bytes of one launch from the committed ncu
 `reference_cuda` = the reference's OWN CUDA pipeline for the same update on the same state, timed in the same
 run (oracle/ref_pipeline.py:RefCudaStep: ref_cuda_corr x2 + stack, torch Update under autocast, ref_cuda_ba
 from oracle/_ref) -- the same-box denominator of north_star's ">= 5x the reference CUDA build".
+`--dump-outputs DIR` writes what the timed path computed in its last timed step (rank 0) as DIR/<name>.npy; the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 `--impl reference` times the reference's CPU path (oracle port of F.grid_sample correlation + PyTorch
 Update + dpvo/ba.py BA, BASELINE.json configs[0] style) on a bounded sample of the same workload.
 """
@@ -275,6 +277,27 @@ def workload_config(config, E):
 
 
 # ------------------------------------------------------------------------------------ GPU path
+DUMP_NET_ROWS = 4096          # rows of the recurrent state kept by --dump-outputs (a fixed seeded sample of E)
+
+
+def step_outputs(st, run, target, weight):
+    """host copies of what one update hands its caller: the BA-refined poses and patch inverse depths of the
+    window, the flow target / confidence of every edge, and a fixed seeded sample of the recurrent state rows"""
+    import torch
+    rows = torch.randperm(st.E, generator=torch.Generator().manual_seed(0))[:DUMP_NET_ROWS].sort().values
+    return {"poses": st.poses[:st.n].float().cpu(), "depths": st.patches[:st.n * run.M, 2, 1, 1].float().cpu(),
+            "target": target[0].float().cpu(), "weight": weight[0].float().cpu(),
+            "net_rows": rows, "net_sample": run.net[0, rows.to(run.net.device)].float().cpu()}
+
+
+def dump_outputs(out_dir, outputs):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in outputs.items():
+        a = v.numpy()
+        np.save(os.path.join(out_dir, k + ".npy"), a.astype(np.float64 if a.dtype.kind in "iu" else np.float32))
+
+
 def run_ours(args):
     import torch
     import dpvo_b200
@@ -316,12 +339,13 @@ def run_ours(args):
     for i in range(args.steps):
         run.timers = {k: v[i] for k, v in ev.items()}
         run.reset()
-        run.step()
+        out = run.step()
     t_end.record()
     barrier()
     windows.append((w0, time.time()))
     launches = ex.launch_count() - l0
     run.timers = None
+    outputs = step_outputs(st, run, *out) if args.dump_outputs and rank == 0 else None
     run.update.gemm_events = None
     gemm_ms = sum(a.elapsed_time(b) for a, b in gemm_events) / args.steps
     gemm_launches = len(gemm_events) // args.steps
@@ -333,6 +357,7 @@ def run_ours(args):
     # ---- the same step as a CUDA graph (how the runner is meant to be driven): timed the same way.  The eager
     # pass above stays for the per-stage breakdown (events cannot be recorded inside a graph).
     launch_mode = "eager launches"
+    graph_out = None
     if not args.no_graph:
         try:
             run.capture()
@@ -343,16 +368,19 @@ def run_ours(args):
             t_start.record()
             for i in range(args.steps):
                 run.reset()
-                run.step_graph()
+                out = run.step_graph()
             t_end.record()
             barrier()
             windows.append((w0, time.time()))
             ms = t_start.elapsed_time(t_end) / args.steps
             launch_mode = "CUDA graph replay (%d kernel nodes per step)" % (launches // args.steps)
             launches *= 2                                  # kernels of the eager pass + of the replays
+            graph_out = out
         except Exception as exc:                           # noqa: BLE001 -- report and keep the eager number
             run.graph = None
             launch_mode = "eager launches (graph capture failed: %s)" % str(exc).splitlines()[0][:120]
+    if outputs is not None and graph_out is not None:      # the reported rate is the graph loop's: dump its last step
+        outputs = step_outputs(st, run, *graph_out)
 
     # ---- end to end: new frame from pinned host memory every step, poses + depths back to host
     hf = run.make_host_frame()
@@ -438,6 +466,8 @@ def run_ours(args):
                              "ncu_source": ncu.get("corr_source")}}
     if not args.no_reference_cuda and world == 1:
         out["reference_cuda"] = reference_cuda_leg(st, run, ms)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
     if not args.no_cpu_baseline and world == 1:          # the CPU leg is timed at N = 1 only
         # same figure as the reference arm reports: one measured update on the whole graph (the strided sample only picks the pool size)
         val, threads, sample, _, _, chk = cpu_reference_measure(args.config, 2, 1, 20.0, full_check=True)
@@ -541,7 +571,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-reference-cuda", action="store_true", help="skip the reference-CUDA-pipeline leg")
     ap.add_argument("--no-graph", action="store_true", help="time eager launches only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, rank 0; --impl ours inference only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.mode == "train" or args.impl == "reference"):
+        ap.error("--dump-outputs writes the outputs of the timed inference step of --impl ours; "
+                 "it is not available with --mode train or --impl reference")
     if args.mode == "train":
         args.steps = 3 if args.steps is None else args.steps
         args.warmup = 1 if args.warmup is None else args.warmup

@@ -51,6 +51,16 @@ def loop_scatter_softmax_sum(fx, gx, key):
     return out
 
 
+def group_rows(x, key):
+    """[1, G, C]: the row of x shared by the edges of each group of `key`, groups in ascending key order;
+    x == group_rows(x, key)[:, inverse] with inverse from torch.unique(key, return_inverse=True)"""
+    _, inv = torch.unique(key, return_inverse=True)
+    first = torch.zeros(int(inv.max()) + 1, dtype=torch.long).scatter_(0, inv.flip(0), torch.arange(key.numel() - 1, -1, -1))
+    rows = x[:, first].clone()
+    assert torch.equal(rows[:, inv], x), "rows differ inside a group"
+    return rows
+
+
 def make_inputs(E, dseed):
     """the seeded inputs of a case (CPU generator: identical on every host); the fixture stores their
     checksums instead of the tensors"""
@@ -80,9 +90,11 @@ def make_case(name):
             agg_loop = mod.agg_ij.h(y)[:, inv]
             assert (agg - agg_loop).abs().max().item() < 1e-5, "scatter stand-in disagrees with the loop definition"
         sums = {k: float(v.double().sum()) for k, v in mod.state_dict().items()}
+    # SoftAgg gives every edge of an (ii, jj) group the same row: store one row per group, in ascending key order
+    agg_rows = group_rows(agg, ii * 12345 + jj)
     return dict(ii=ii, jj=jj, kk=kk, weight_seed=wseed, data_seed=dseed,
                 input_sums=[float(t.double().sum()) for t in (net, inp, corr, x)],
-                out_net=out_net, out_delta=delta, out_weight=weight, softagg_out=agg,
+                out_net=out_net, out_delta=delta, out_weight=weight, softagg_rows=agg_rows,
                 param_sums=sums, source="dpvo/net.py:Update + dpvo/blocks.py (reference, imported unmodified), fp32 CPU, torch %s" % torch.__version__)
 
 

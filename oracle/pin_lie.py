@@ -1,8 +1,10 @@
 """ORACLE pinning (test infrastructure): run the reference's OWN lietorch test functions
-(dpvo/lietorch/run_tests.py:16-226, unmodified, imported from /root/reference) with the CPU
-restatement oracle/lie.py standing in for the native `lietorch_backends` module.
+(dpvo/lietorch/run_tests.py:16-226, unmodified) with the CPU restatement oracle/lie.py standing in for
+the native `lietorch_backends` module.
 
-Only possible where /root/reference is mounted (the build container).  Covers SO3, RxSO3, SE3 and Sim3
+The files are imported from the reference tree where it is mounted, else from the copy of the reference's
+Python package that oracle/build_ref.py:stage_python packs into oracle/_ref/dpvo_ref_py.zip
+(`available()` says whether either is there).  Covers SO3, RxSO3, SE3 and Sim3
 (`groups` selects; the product kernels implement SO3 and SE3): the
 forward identities at atol 1e-8 in fp64 and the analytic-vs-numeric Jacobian checks of the backward
 operators.  Usage: python oracle/pin_lie.py   (exit code 0 = pinned)
@@ -13,13 +15,28 @@ import sys
 
 REF = "/root/reference/dpvo"
 HERE = os.path.dirname(os.path.abspath(__file__))
+REF_ZIP = os.path.join(HERE, "_ref", "dpvo_ref_py.zip")
+
+
+def _ref_dir():
+    """the reference's dpvo/ package: the mounted tree, else its staged copy (a zip on sys.path is importable)"""
+    if os.path.isdir(REF):
+        return REF
+    if os.path.exists(REF_ZIP):
+        return REF_ZIP + "/dpvo"
+    return None
+
+
+def available():
+    return _ref_dir() is not None
 
 
 def run(verbose=True, groups=("SO3", "SE3")):
-    if not os.path.isdir(REF):
-        raise RuntimeError("reference tree not mounted at %s" % REF)
+    ref = _ref_dir()
+    if ref is None:
+        raise RuntimeError("reference package found neither at %s nor staged at %s" % (REF, REF_ZIP))
     saved = list(sys.path)
-    sys.path[:0] = [os.path.join(HERE, "shims"), os.path.join(REF, "lietorch"), REF]
+    sys.path[:0] = [os.path.join(HERE, "shims"), ref + "/lietorch", ref]
     for m in ("lietorch", "lietorch_backends", "gradcheck", "run_tests"):
         sys.modules.pop(m, None)
     try:

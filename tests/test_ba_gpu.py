@@ -3,6 +3,7 @@ inverse depths within 1e-4 relative."""
 import pytest
 import torch
 
+import refdata
 from oracle import ba as OB
 from dpvo_b200 import synthetic
 
@@ -181,20 +182,25 @@ def test_ba_wide_window_and_eff_impl_match_oracle_and_reference_kernel(ext, ref_
     lm = torch.tensor([1e-4])
     rp, rq = OB.fastba_forward(st.poses.double(), st.patches.double(), st.intrinsics.double(), target.double(), weight.double(),
                                lm.double(), st.ii, st.jj, st.kk, t0, st.n, 2)
-    outs = []
-    for mod in ([ext[1]] + ([ref_ext[1]] if ref_ext is not None else [])):
+    live = st.kk.unique()
+
+    def run(mod):
         poses, patches = st.poses.clone().to(DEV)[None], st.patches.clone().to(DEV)[None]
         mod.forward(poses, patches, st.intrinsics.to(DEV)[None], target.to(DEV)[None], weight.to(DEV)[None], lm.to(DEV),
                     st.ii.to(DEV), st.jj.to(DEV), st.kk.to(DEV), st.cfg["M"], t0, st.n, 2, eff_impl)
-        outs.append((poses[0, :st.n].cpu().double(), patches[0].cpu().double()))
-    live = st.kk.unique()
+        return poses[0, :st.n].cpu().double(), patches[0].cpu().double()[live, 2]
+
+    ours = run(ext[1])
+    R = refdata.reference("ba_wide_%s_t%d" % ("eff" if eff_impl else "dense", t0), ref_ext,
+                          lambda rx: dict(zip(("poses", "depth"), run(rx[1]))))
     assert st.n - t0 > 32 or eff_impl
-    for p, q in outs:
-        assert torch.isfinite(p).all() and torch.isfinite(q[live]).all()
-        assert _rel(p, rp[:st.n]) < 1e-4 and _rel(q[live, 2], rq[live, 2]) < 1e-4
-    assert (outs[0][0] - st.poses[:st.n].double()).abs().max().item() > 1e-4      # the step moved the poses
+    for p, q, pick in ((ours[0], ours[1], lambda x: x), (R["poses"].double(), R["depth"].double(), lambda x: R.pick("depth", x))):
+        assert torch.isfinite(p).all() and torch.isfinite(q).all()
+        assert _rel(p, rp[:st.n]) < 1e-4
+        assert ((q - pick(rq[live, 2])).abs().max() / rq[live, 2].abs().max()).item() < 1e-4
+    assert (ours[0] - st.poses[:st.n].double()).abs().max().item() > 1e-4      # the step moved the poses
     if t0 > 1:
-        assert torch.equal(outs[0][0][:t0].float(), st.poses[:t0])                 # poses before t0 stay fixed
+        assert torch.equal(ours[0][:t0].float(), st.poses[:t0])                 # poses before t0 stay fixed
 
 
 def test_ba_wide_rejects_patch_ids_outside_their_frame(ext):

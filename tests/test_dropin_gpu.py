@@ -11,6 +11,7 @@ import sys
 import pytest
 import torch
 
+import refdata
 from oracle import ba as OB, corr as OC, refimport
 from dpvo_b200 import synthetic
 
@@ -150,35 +151,55 @@ def test_reference_transform_jacobians_on_our_lietorch(refpy):
 
 
 @pytest.mark.parametrize("config,n_frames", [("fast", 14)])
-def test_reference_update_module_vs_ours_same_weights(refpy, ext, config, n_frames):
+def test_reference_update_module_vs_ours_same_weights(ext, config, n_frames):
     """dpvo/net.py:Update (torch, autocast as dpvo.py:332, calling OUR cuda_ba.neighbors) vs dpvo_b200.net.Update
     (tcgen05) with the same state_dict, both against the reference module in fp32: ours no worse than 2x the
-    reference's own mixed-precision error"""
+    reference's own mixed-precision error.  The reference module runs live where its package is staged, else its
+    stored outputs stand in (tests/refdata.py); either way ours is also held, on every element, to the fp32
+    restatement oracle/update.py with the same weights."""
     from dpvo_b200.net import Update
+    from oracle import update as OU
     st = synthetic.make_state(config, n_frames, device="cpu", features=False)
     E = st.E
     torch.manual_seed(1234)
-    ref_mod = refpy["net"].Update(3).to(DEV).eval()
+    weights = OU.Update(3).state_dict()              # net.py:28-72 construction order: the reference module's seeded weights
     ours = Update(3).to(DEV).eval()
-    ours.load_state_dict(ref_mod.state_dict())
+    ours.load_state_dict(weights)
+    mod32 = OU.Update(3).to(DEV).eval()
+    mod32.load_state_dict(weights)
     g = torch.Generator().manual_seed(64)
     net = (torch.randn(1, E, 384, generator=g) * 0.5).to(DEV)
     inp = (torch.randn(1, E, 384, generator=g) * 0.25).half().to(DEV)
     corr = (torch.randn(1, E, 882, generator=g) * 2).half().to(DEV)
     ii, jj, kk = st.ii.to(DEV), st.jj.to(DEV), st.kk.to(DEV)
-    with torch.no_grad():
-        rn, (rd, rw, _) = ref_mod(net, inp.float(), corr.float(), None, ii, jj, kk)
-        with torch.autocast("cuda", dtype=torch.half):
-            an, (ad, aw, _) = ref_mod(net, inp, corr, None, ii, jj, kk)
-        on, (od, ow, _) = ours(net, inp, corr, None, ii, jj, kk)
 
     def err(a, b):
         return (a.float() - b.float()).abs().max().item()
 
-    print("ours vs fp32:", err(on, rn), err(od, rd), err(ow, rw), " autocast vs fp32:", err(an, rn), err(ad, rd), err(aw, rw))
-    assert err(on, rn) <= max(2 * err(an, rn), 2e-2)
-    assert err(od, rd) <= max(2 * err(ad, rd), 1e-2)
-    assert err(ow, rw) <= max(2 * err(aw, rw), 5e-3)
+    def compute(_):
+        with refimport.reference_python(native=ext[:3]):
+            import dpvo.net as RN
+            ref_mod = RN.Update(3).to(DEV).eval()
+            ref_mod.load_state_dict(weights)
+            with torch.no_grad():
+                rn, (rd, rw, _) = ref_mod(net, inp.float(), corr.float(), None, ii, jj, kk)
+                with torch.autocast("cuda", dtype=torch.half):
+                    an, (ad, aw, _) = ref_mod(net, inp, corr, None, ii, jj, kk)
+        return dict(net=rn.float(), delta=rd.float(), weight=rw.float(),
+                    autocast_err_net=err(an, rn), autocast_err_delta=err(ad, rd), autocast_err_weight=err(aw, rw))
+
+    R = refdata.reference("update_module_%s%d" % (config, n_frames), refimport if refimport.staged() else None, compute)
+    with torch.no_grad():
+        on, (od, ow, _) = ours(net, inp, corr, None, ii, jj, kk)
+        n32, (d32, w32, _) = mod32(net, inp.float(), corr.float(), None, ii, jj, kk)
+
+    mine = {"net": on, "delta": od, "weight": ow}
+    e = {k: err(R.pick(k, mine[k]), R[k].to(DEV)) for k in mine}
+    print("ours vs fp32:", e["net"], e["delta"], e["weight"],
+          " autocast vs fp32:", R["autocast_err_net"], R["autocast_err_delta"], R["autocast_err_weight"])
+    for k, o32, bar in (("net", n32, 2e-2), ("delta", d32, 1e-2), ("weight", w32, 5e-3)):
+        assert e[k] <= max(2 * R["autocast_err_" + k], bar), k
+        assert err(mine[k], o32) <= max(2 * R["autocast_err_" + k], bar), k
 
 
 # ------------------------------------------------------------------------------ the whole DPVO class

@@ -2,7 +2,6 @@
 oracle's lietorch_backends stand-in (oracle/shims) monkeypatched under dpvo_b200.lietorch."""
 import importlib.util
 import os
-import sys
 
 import pytest
 
@@ -11,8 +10,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 
 @pytest.fixture()
 def gpu_tests(monkeypatch):
-    sys.path.insert(0, os.path.join(HERE, "..", "oracle", "shims"))
-    import lietorch_backends as LB
+    from oracle import lietorch_backend
+    LB = lietorch_backend()
     import dpvo_b200.lietorch.groups as Gm
     import dpvo_b200.projective_ops as pops
     monkeypatch.setattr(Gm, "_B", LB)
@@ -22,7 +21,6 @@ def gpu_tests(monkeypatch):
     spec.loader.exec_module(m)
     m.DEV = "cpu"
     yield m
-    sys.path.pop(0)
 
 
 @pytest.mark.parametrize("name", ["test_transform_and_jacobians_match_oracle", "test_transform_autograd_matches_oracle_autograd",

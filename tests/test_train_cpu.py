@@ -1,16 +1,12 @@
 """Training-path host code without a GPU: the differentiable bundle adjustment of dpvo_b200/ba.py against the
-REFERENCE's own dpvo/ba.py:BA (imported unmodified from /root/reference, lietorch served by the CPU oracle on
-both sides), outputs and gradients in fp64; and the sequence loss on a hand-checkable case."""
-import os
-import sys
-
+REFERENCE's own dpvo/ba.py:BA (imported unmodified from the reference sources where they are at hand, else its
+stored outputs; lietorch served by the CPU oracle on both sides), outputs and gradients in fp64; and the sequence loss on a hand-checkable case."""
 import pytest
 import torch
 
+import refdata
 from oracle import refimport
 from dpvo_b200 import synthetic
-
-HERE = os.path.dirname(os.path.abspath(__file__))
 
 
 class _UniqueGroups:
@@ -23,14 +19,13 @@ class _UniqueGroups:
 
 @pytest.fixture()
 def cpu_ops(monkeypatch):
-    sys.path.insert(0, os.path.join(HERE, "..", "oracle", "shims"))
-    import lietorch_backends as LB
+    from oracle import lietorch_backend
+    LB = lietorch_backend()
     import dpvo_b200.lietorch.groups as Gm
     import dpvo_b200.ba as ba
     monkeypatch.setattr(Gm, "_B", LB)
     monkeypatch.setattr(ba, "EdgeGroups", _UniqueGroups)
     yield ba
-    sys.path.pop(0)
 
 
 def _problem(seed, structure_only=False):
@@ -47,13 +42,12 @@ def _problem(seed, structure_only=False):
     return st, poses, patches, intr, target, weight
 
 
-@pytest.mark.skipif(not refimport.available(), reason="/root/reference not mounted")
 @pytest.mark.parametrize("structure_only", [False, True])
 def test_differentiable_ba_matches_the_reference_ba_forward_and_backward(cpu_ops, structure_only):
     from dpvo_b200.lietorch import SE3
     st, poses, patches, intr, target, weight = _problem(3)
     bounds = [-64, -64, 80 + 64, 60 + 64]
-    h, w = 60, 80
+    names = ("poses", "patches", "d/dtarget", "d/dweight", "d/dpatches")
 
     def run(BA, SE3cls, lm):
         t = target.clone().requires_grad_(True)
@@ -70,13 +64,17 @@ def test_differentiable_ba_matches_the_reference_ba_forward_and_backward(cpu_ops
         return G.data.detach(), Q.detach(), gt, gw, gq
 
     mine = run(cpu_ops.BA, SE3, 1e-4)
-    with refimport.reference_modules():
-        import dpvo.ba as RB
-        from dpvo.lietorch import SE3 as RSE3
-        theirs = run(RB.BA, RSE3, 1e-4)
-    for a, b, nm in zip(mine, theirs, ("poses", "patches", "d/dtarget", "d/dweight", "d/dpatches")):
-        scale = max(1.0, b.abs().max().item())
-        assert (a - b).abs().max().item() <= 1e-8 * scale, (nm, (a - b).abs().max().item())
+
+    def compute(_):
+        with refimport.reference_modules():
+            import dpvo.ba as RB
+            from dpvo.lietorch import SE3 as RSE3
+            return dict(zip(names, run(RB.BA, RSE3, 1e-4)))
+
+    R = refdata.reference("train_ba_%s" % ("structure" if structure_only else "full"), refimport if refimport.available() else None, compute)
+    for a, nm in zip(mine, names):
+        scale = max(1.0, R.absmax(nm))
+        assert (R.pick(nm, a) - R[nm]).abs().max().item() <= 1e-8 * scale, (nm, (R.pick(nm, a) - R[nm]).abs().max().item())
     if not structure_only:
         assert (mine[0] - poses).abs().max().item() > 1e-4          # the step moved the poses
 
